@@ -2356,6 +2356,11 @@ static int32_t rank_bench_decode(b200rwkv_engine* e, int32_t nslot, const int32_
     }
     CK(cudaEventRecord(eb, e->stream));
     CK(cudaStreamSynchronize(e->stream));
+    {
+        // every step kept each slot's logits row in HBM (enqueue_keep): readable as after b200rwkv_infer(logits_out = NULL)
+        std::lock_guard<std::mutex> lk2(e->keep_mu);
+        for (int i = 0; i < nslot; ++i) e->keep_valid[slot[i]] = 1;
+    }
     CK(cudaEventElapsedTime(ms_out, ea, eb));
     for (int i = 0; i < (int)marks.size(); ++i) {
         CK(cudaEventElapsedTime(step_ms_out + i, i == 0 ? ea : marks[i - 1], marks[i]));

@@ -16,6 +16,11 @@ there are no checkpoints offline).
   cpu_baseline / --impl reference
             the C/OpenMP oracle (oracle/rwkv_ref.c) on the host cores, same weights/tokens
             (the reference's own web-rwkv+lavapipe path cannot be built here: no Rust, no Vulkan)
+
+--dump-outputs DIR writes what the timed path computed in its last step as DIR/<name>.npy (f32), so two builds can be
+compared output for output on identical seeded inputs: decode -> `logits` [batch, vocab] and `state` [batch, L, N+2, C],
+prefill -> `state` of every sequence.  An array over its share of DUMP_BYTES is replaced by a fixed seeded sample of its
+flattened elements.
 """
 from __future__ import annotations
 
@@ -106,6 +111,33 @@ def make_tokens(n_steps: int, batch: int, vocab: int):
     return rng.integers(1, min(vocab, 65530), size=(batch, n_steps), dtype=np.int64)
 
 
+DUMP_BYTES = 48 << 20          # all of --dump-outputs together, .npy headers aside
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a, np.float32)
+        if a.nbytes > share:
+            a = a.reshape(-1)[np.unique(np.random.default_rng(0).integers(0, a.size, share // a.itemsize))]
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
+def last_step_outputs(model, slots) -> dict:
+    """Logits row and state of every slot after the model's most recent step, through device snapshots (untimed)."""
+    logits = np.empty((len(slots), model.info["num_vocab"]), np.float32)
+    state = None
+    for i, s in enumerate(slots):
+        snap = model.state.read(s)
+        st, logits[i] = model.state.snapshot_back(snap, with_logits=True)
+        snap.free()
+        if state is None:
+            state = np.empty((len(slots),) + st.shape, np.float32)
+        state[i] = st
+    return {"logits": logits, "state": state}
+
+
 def host_threads() -> int:
     """Threads the CPU arms use: the physical cores inside this process' affinity mask and cgroup CPU quota (measured on
     the GPU box: 128 OpenMP threads on its 64 cores run the same step 18x slower than 64).  Never taken from
@@ -165,7 +197,7 @@ def prefill_main(args):
     preset = args.preset if args.preset != "v6-7b" or "--preset" in sys.argv else "v6-3b"
     shape = synth.PRESETS[preset]
     B, Tn = args.seqs, args.seq_len
-    steps, warm = max(1, min(args.steps, 4)), max(3, args.warmup if args.warmup < 8 else 3)
+    steps, warm = args.steps, max(3, args.warmup if args.warmup < 8 else 3)
     metric = f"prefill tokens/s {MODEL_NAMES.get(preset, preset)} fp16 {B}x{Tn}-token inputs (embeddings route)"
     st = synth.make_st(shape, 0)
     PASS = 128                                              # tokens per weight pass (the engine's largest step)
@@ -201,6 +233,8 @@ def prefill_main(args):
         t_dev.append(t1 - t0); t_e2e.append(t2 - t0)
     clocks = sampler.stop()
     launches = model.launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"state": state_buf})
     ntok = B * Tn
     dt, de = float(np.mean(t_dev)), float(np.mean(t_e2e))
     checksum = [float(state_buf.astype(np.float64).sum()), float(np.abs(state_buf).astype(np.float64).sum())]
@@ -284,7 +318,7 @@ def main():
     global PRESET, BATCH
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=128)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 128 decode steps, 4 prefill passes)")
     ap.add_argument("--warmup", type=int, default=8)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--cpu-steps", type=int, default=int(os.environ.get("B200RWKV_BENCH_CPU_STEPS", "6")))
@@ -298,7 +332,12 @@ def main():
     ap.add_argument("--quant-layers", type=int, default=-1, help="the reference's `quant`: first N layers (default: all)")
     ap.add_argument("--seqs", type=int, default=256)
     ap.add_argument("--seq-len", type=int, default=512)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (1-GPU B200 arm)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 4 if args.mode == "prefill" else 128
+    assert args.steps >= 1, "--steps must be at least 1"
     args.warmup = max(args.warmup, 3)
     PRESET, BATCH = args.preset, args.batch
     METRIC = metric_name(PRESET, BATCH)
@@ -311,6 +350,7 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    assert not args.dump_outputs or (args.impl == "b200" and world == 1), "--dump-outputs: 1-GPU B200 arm only"
 
     from ai00_server_b200 import synth
     from oracle import rwkv_numpy as O          # only for parse_st of the cpu arm (checker side)
@@ -383,6 +423,8 @@ def main():
     ms, launches = model.bench_decode(slots, dec, args.warmup, args.steps)
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_step_outputs(model, slots))
     if world > 1:
         t = torch.tensor([ms], device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

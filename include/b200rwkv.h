@@ -204,7 +204,8 @@ void b200rwkv_host_free(void* p);
 /* Measurement hook used by bench.py for the kernel-resident number: runs `warmup + steps`
  * decode steps (one token per listed slot per step) with token ids staged in HBM beforehand,
  * no host<->device traffic inside the timed region; returns CUDA-event milliseconds for the
- * `steps` timed steps and the number of kernel launches in that region. */
+ * `steps` timed steps and the number of kernel launches in that region.  The last logits row of
+ * every listed slot stays in HBM as after b200rwkv_infer with logits_out = NULL. */
 int32_t b200rwkv_bench_decode(b200rwkv_engine*, int32_t nslot, const int32_t* slot,
                               const uint32_t* tokens /* [(warmup+steps) * nslot] */, int32_t warmup,
                               int32_t steps, int32_t flush_l2, float* ms_out, int64_t* launches_out,
