@@ -18,6 +18,7 @@ OK = 0
 ERR_INVALID, ERR_UNSUPPORTED, ERR_CUDA, ERR_STATE = -1, -2, -3, -4
 OPTION_LAST, OPTION_FULL, OPTION_NONE = 0, 1, 2
 TP_HANDLE_BYTES = 128
+PLAN_INTS = 48            # B200RWKV_PLAN_INTS: one b200rwkv_debug_plan record
 
 
 class Info(C.Structure):
@@ -85,7 +86,8 @@ SYMBOLS = [
     ("b200rwkv_launch_count", C.c_int32, [_P, C.POINTER(C.c_int64)]),
     ("b200rwkv_keep_hidden", C.c_int32, [_P, C.c_int32]),
     ("b200rwkv_last_hidden", C.c_int32, [_P, _P, C.c_size_t]),
-    ("b200rwkv_debug_read", C.c_int32, [_P, C.c_char_p, _P, C.c_size_t]),
+    ("b200rwkv_debug_read", C.c_int32, [_P, C.c_char_p, _P, C.c_size_t, C.POINTER(C.c_int32)]),
+    ("b200rwkv_debug_plan", C.c_int32, [_P, C.c_int32, C.c_int32, _P, C.c_size_t]),
     ("b200rwkv_debug_trace", C.c_int32, [_P, _P, C.c_size_t, _P, _P]),
     ("b200rwkv_debug_gemm_time", C.c_int32, [_P, C.c_int32, C.c_int32, C.POINTER(C.c_float), C.POINTER(C.c_int64), _P]),
     ("b200rwkv_last_error", C.c_char_p, [_P]),

@@ -350,6 +350,7 @@ struct GemmLaunch {
     int total_tiles = 0;
     size_t weight_bytes = 0;   // algorithmic (unpadded) weight bytes streamed (f16, or codes + block parameters)
     int qtype = QT_NONE;       // weight format of every segment of the launch (qgemm.cuh)
+    bool forced = false;       // grid fixed by the caller (static split-K: tiles x slices CTAs)
 };
 
 struct SegDesc {
@@ -467,7 +468,10 @@ struct b200rwkv_engine {
     std::map<int, long long> graph_launches;   // kernels per captured step graph
     long long launch_total = 0;                // kernels launched by this engine's steps since creation
     long long launches_last_step = 0;
-    int last_T = 0, last_th = 16;      // tokens / A16 token rows of the most recent step
+    // the most recent step of b200rwkv_infer (b200rwkv_debug_read): tokens, output rows, token rows of the A16 operands and
+    // of the head's operand, split (hi + lo) operands
+    int last_T = 0, last_R = 0, last_th = 16, last_th_rows = 16;
+    bool last_split = false;
 
     // softmax
     float *sm_in = nullptr, *sm_out = nullptr;
@@ -538,6 +542,7 @@ struct b200rwkv_engine {
     }
     void launch_gemm(const GemmLaunch& g, int MT, cudaStream_t s, Profiler* prof, bool split = false);
     void enqueue_step(cudaStream_t s, int MT, int MTR, Profiler* prof);
+    bool pre_skipped(const Layer& ly, int gi, int MT) const;
     void run_step(int MT, int MTR);
     int fill_meta(int* m, const std::vector<int>& slots, const std::vector<int>& counts, const std::vector<const uint32_t*>& toks,
                   const std::vector<int>& outmode /*0 none,1 last,2 full*/, int* R_out);
@@ -674,6 +679,7 @@ GemmLaunch b200rwkv_engine::make_launch(std::vector<SegDesc>& segs, int force_gr
     GemmLaunch g;
     memset(&g.p, 0, sizeof(g.p));
     g.qtype = qtype;
+    g.forced = force_grid > 0;
     g.p.qvar = 1;
     if (const char* v = dbg_env("B200RWKV_QVAR")) g.p.qvar = atoi(v);
     const size_t blk_bytes = (size_t)q_block_bytes(qtype);
@@ -1347,17 +1353,17 @@ void b200rwkv_engine::finalize_tp() {
 // -----------------------------------------------------------------------------------------
 // one forward step over the tokens described by d_meta
 // -----------------------------------------------------------------------------------------
+bool b200rwkv_engine::pre_skipped(const Layer& ly, int gi, int MT) const {
+    if (fold_wd2 && gi == ly.wd2_index) return true;                 // the WKV kernel evaluates the decay LoRA stage 2
+    return fused_pre_ok && MT == 1 && ly.w1_raw && gi < 2;           // the front-half kernel holds both ddlerp LoRA stages
+}
+
 void b200rwkv_engine::enqueue_step(cudaStream_t s, int MT, int MTR, Profiler* prof) {
     launches_last_step = 0;
     const int rows = MT * 16;
     // token rows of this step's A16 operands (common.cuh): every producer and consumer of the step uses the same value
     const int th = (split_on && MT == 1) ? 32 : 16 * MT;
     const int th_rows = (split_on && MT == 1) ? 32 : 16 * MTR;        // the head's operand holds output rows
-    last_th = th;
-    auto pre_skipped = [&](const Layer& ly, int gi) {
-        if (fold_wd2 && gi == ly.wd2_index) return true;                 // the WKV kernel evaluates the decay LoRA stage 2
-        return fused_pre_ok && MT == 1 && ly.w1_raw && gi < 2;           // the front-half kernel holds both ddlerp LoRA stages
-    };
     // projection launches of this step in stream order: each one prefetches the head of the next into L2 (the last one
     // wraps around to the first launch of the next step)
     std::vector<const GemmLaunch*> seq;
@@ -1365,7 +1371,7 @@ void b200rwkv_engine::enqueue_step(cudaStream_t s, int MT, int MTR, Profiler* pr
         for (int l = 0; l < L; ++l) {
             const Layer& ly = layers[l];
             for (int gi = 0; gi < (int)ly.pre.size(); ++gi)
-                if (!pre_skipped(ly, gi)) seq.push_back(&ly.pre[gi]);
+                if (!pre_skipped(ly, gi, MT)) seq.push_back(&ly.pre[gi]);
             seq.push_back(&ly.o);
             for (auto& g : ly.ffn) seq.push_back(&g);
         }
@@ -1434,7 +1440,7 @@ void b200rwkv_engine::enqueue_step(cudaStream_t s, int MT, int MTR, Profiler* pr
             launch_ln(ly.ln1);
         }
         for (int gi = 0; gi < (int)ly.pre.size(); ++gi)
-            if (!pre_skipped(ly, gi)) gemm(ly.pre[gi]);
+            if (!pre_skipped(ly, gi, MT)) gemm(ly.pre[gi]);
         {
             // decays / staged rows are sized by the step shape: a slot cannot hold more tokens than the step
             WkvParams wp = ly.wkv;
@@ -1482,6 +1488,10 @@ void b200rwkv_engine::enqueue_keep(cudaStream_t s, int MTR) {
 }
 
 void b200rwkv_engine::run_step(int MT, int MTR) {
+    // recorded here, not in enqueue_step: a replayed graph does not enqueue again (same formulas as enqueue_step)
+    last_split = split_on && MT == 1;
+    last_th = last_split ? 32 : 16 * MT;
+    last_th_rows = last_split ? 32 : 16 * MTR;
     if (!use_graph) {
         enqueue_step(stream, MT, MTR, nullptr);
         enqueue_keep(stream, MTR);
@@ -1628,6 +1638,7 @@ void b200rwkv_engine::infer(int nslot, const int32_t* slot, const int32_t* ntok,
         int R = 0;
         const int T = fill_meta(hm, s_slots, s_counts, s_toks, s_out, &R);
         last_T = T;
+        last_R = R;
         CK(cudaMemcpyAsync(d_meta, hm, meta_ints * 4, cudaMemcpyHostToDevice, stream));
         CK(cudaEventRecord(meta_ev[mb], stream));
         run_step(mt_bucket(T), R > 0 ? mt_bucket(R) : 0);
@@ -2641,11 +2652,12 @@ int32_t b200rwkv_last_hidden(b200rwkv_engine* e, float* out, size_t cap) {
     return st < 0 ? st : rows;
 }
 
-// Debug aid for the parity tests: copy a named internal activation buffer of the most recent
-// step to the host as f32 row-major [rows, cols]; returns cols (rows = tokens of the last step,
-// capped by `cap`), or a negative status.  Not used on the product path.
-int32_t b200rwkv_debug_read(b200rwkv_engine* e, const char* name, float* out, size_t cap) {
-    if (!e || !name || !out) return B200RWKV_ERR_INVALID;
+// Test aid: copy a named internal activation buffer of the most recent step of b200rwkv_infer to the host as f32 row-major
+// [rows, cols]; returns cols and stores rows (the step's tokens; output rows for `a_head`), or a negative status.  A16 buffers
+// of a split-operand step hold hi values in token rows 0..15 and lo values in rows 16..31: they are returned as hi + lo, the
+// value the projection consumes (exact in f32).  Not used on the product path.
+int32_t b200rwkv_debug_read(b200rwkv_engine* e, const char* name, float* out, size_t cap, int32_t* rows_out) {
+    if (!e || !name || !out || !rows_out) return B200RWKV_ERR_INVALID;
     std::string* errp_ = &g_err;
     try {
         std::lock_guard<std::mutex> lk(e->mu);
@@ -2668,6 +2680,7 @@ int32_t b200rwkv_debug_read(b200rwkv_engine* e, const char* name, float* out, si
                     CK(cudaMemcpy(tmp.data(), f.p + (size_t)sp * e->maxT * e->C, tmp.size() * 4, cudaMemcpyDeviceToHost));
                     for (size_t i = 0; i < tmp.size(); ++i) out[i] += tmp[i];
                 }
+                *rows_out = T;
                 return f.cols;
             }
         struct A { std::string n; const A16Buf* b; int cols; int mat; };
@@ -2680,11 +2693,18 @@ int32_t b200rwkv_debug_read(b200rwkv_engine* e, const char* name, float* out, si
         as.push_back({"a_head", &e->a_head, e->C, 0});
         for (const A& a : as)
             if (n == a.n && a.b->p) {
-                REQUIRE((size_t)T * a.cols <= cap, B200RWKV_ERR_INVALID, "debug buffer too small");
+                const bool head = (n == "a_head");        // the head's operand holds output rows (R), not tokens
+                const int rows = head ? e->last_R : T, th = head ? e->last_th_rows : e->last_th;
+                REQUIRE((size_t)rows * a.cols <= cap, B200RWKV_ERR_INVALID, "debug buffer too small");
                 std::vector<__half> h(a.b->halves_per_matrix);
                 CK(cudaMemcpy(h.data(), a.b->p + (size_t)a.mat * a.b->halves_per_matrix, h.size() * 2, cudaMemcpyDeviceToHost));
-                for (int t = 0; t < T; ++t)
-                    for (int c = 0; c < a.cols; ++c) out[(size_t)t * a.cols + c] = __half2float(h[a16_index(t, c, e->last_th)]);
+                for (int t = 0; t < rows; ++t)
+                    for (int c = 0; c < a.cols; ++c) {
+                        float v = __half2float(h[a16_index(t, c, th)]);
+                        if (e->last_split) v += __half2float(h[a16_index(t + 16, c, th)]);
+                        out[(size_t)t * a.cols + c] = v;
+                    }
+                *rows_out = rows;
                 return a.cols;
             }
         throw Error(B200RWKV_ERR_INVALID, "unknown debug buffer: " + n);
@@ -2698,6 +2718,46 @@ int32_t b200rwkv_debug_read(b200rwkv_engine* e, const char* name, float* out, si
         *errp_ = "unknown exception";
         return B200RWKV_ERR_INVALID;
     }
+}
+
+// Test aid: the projection launches a step of MT token tiles runs for layer `layer` (-1: the head, at MT output-row tiles), in
+// stream order; one record of B200RWKV_PLAN_INTS int32 each (layout in include/b200rwkv.h).  Returns the number of launches.
+static_assert(B200RWKV_PLAN_INTS == 8 + 5 * GEMM_MAX_SEG, "plan record layout");
+int32_t b200rwkv_debug_plan(b200rwkv_engine* e, int32_t layer, int32_t mt, int32_t* out, size_t cap) {
+    int32_t count = 0;
+    const int32_t st = [&]() -> int32_t {
+        API_BEGIN(e)
+        REQUIRE(e && out, B200RWKV_ERR_INVALID, "null argument");
+        REQUIRE(layer >= -1 && layer < e->L, B200RWKV_ERR_INVALID, "debug_plan: layer out of range");
+        REQUIRE(mt == 1 || mt == 2 || mt == 4 || mt == 8, B200RWKV_ERR_INVALID, "debug_plan: mt must be 1, 2, 4 or 8");
+        std::lock_guard<std::mutex> lk(e->mu);
+        std::vector<const GemmLaunch*> gs;
+        if (layer < 0) {
+            gs.push_back(&e->head);
+        } else {
+            const Layer& ly = e->layers[layer];
+            for (int gi = 0; gi < (int)ly.pre.size(); ++gi)
+                if (!e->pre_skipped(ly, gi, mt)) gs.push_back(&ly.pre[gi]);
+            gs.push_back(&ly.o);
+            for (auto& g : ly.ffn) gs.push_back(&g);
+        }
+        REQUIRE(gs.size() * B200RWKV_PLAN_INTS <= cap, B200RWKV_ERR_INVALID, "debug_plan: buffer too small");
+        for (const GemmLaunch* g : gs) {
+            int32_t* r = out + (size_t)count * B200RWKV_PLAN_INTS;
+            memset(r, 0, B200RWKV_PLAN_INTS * 4);
+            r[0] = mt >= 4 ? g->grid_wide : g->grid;         // launch_gemm: split-operand decode steps run `grid` too
+            r[1] = g->grid; r[2] = g->grid_wide; r[3] = g->p.total_blocks; r[4] = g->p.max_contrib; r[5] = g->qtype;
+            r[6] = g->forced ? 1 : 0; r[7] = g->p.nseg;
+            for (int i = 0; i < g->p.nseg; ++i) {
+                const GemmSeg& sg = g->p.seg[i];
+                int32_t* q = r + 8 + 5 * i;
+                q[0] = sg.KB; q[1] = sg.tiles; q[2] = sg.N; q[3] = sg.out_mode; q[4] = sg.act;
+            }
+            ++count;
+        }
+        API_END
+    }();
+    return st < 0 ? st : count;
 }
 
 // Profiling aid: the raw stamp rows of the most recent traced replay (b200rwkv_profile_insitu): one row of 512 uint64 per

@@ -373,11 +373,25 @@ class Model:
         capi.check(r, self._h)
         return buf[:r]
 
-    def debug_read(self, name: str, rows: int = 64) -> np.ndarray:
-        buf = np.empty(rows * 65536, np.float32)
-        cols = capi.lib().b200rwkv_debug_read(self._h, name.encode(), capi.ptr(buf), buf.size)
+    def debug_read(self, name: str) -> np.ndarray:
+        """A named activation buffer of the most recent internal step (b200rwkv_debug_read): [rows, cols] f32, rows as the
+        engine reports them (the step's tokens; its output rows for "a_head")."""
+        buf = np.empty(128 * 65536, np.float32)
+        rows = C.c_int32(0)
+        cols = capi.lib().b200rwkv_debug_read(self._h, name.encode(), capi.ptr(buf), buf.size, C.byref(rows))
         capi.check(cols, self._h)
-        return buf[: rows * cols].reshape(rows, cols)
+        return buf[: rows.value * cols].reshape(rows.value, cols).copy()
+
+    def debug_plan(self, layer: int, mt: int) -> list[dict]:
+        """Projection launches of `layer` (-1: the head) in a step of `mt` token tiles (b200rwkv_debug_plan)."""
+        buf = np.zeros(64 * capi.PLAN_INTS, np.int32)
+        n = capi.check(capi.lib().b200rwkv_debug_plan(self._h, layer, mt, capi.ptr(buf), buf.size), self._h)
+        out = []
+        for r in buf[: n * capi.PLAN_INTS].reshape(n, capi.PLAN_INTS):
+            segs = [dict(zip(("KB", "tiles", "N", "out_mode", "act"), (int(x) for x in r[8 + 5 * i: 13 + 5 * i]))) for i in range(r[7])]
+            out.append(dict(grid_run=int(r[0]), grid=int(r[1]), grid_wide=int(r[2]), total_blocks=int(r[3]), max_contrib=int(r[4]),
+                            qtype=int(r[5]), forced=bool(r[6]), segs=segs))
+        return out
 
     def bench_decode(self, slots, tokens: np.ndarray, warmup: int, steps: int, flush_l2: bool = False):
         a_slot = np.asarray(slots, np.int32)

@@ -255,9 +255,20 @@ int32_t b200rwkv_launch_count(b200rwkv_engine*, int64_t* total);
 int32_t b200rwkv_keep_hidden(b200rwkv_engine*, int32_t enable);
 int32_t b200rwkv_last_hidden(b200rwkv_engine*, float* out, size_t cap);
 
-/* Test aid: copy a named internal activation buffer of the most recent step to the host as f32
- * row-major; returns the column count (negative status on error).  Not on the product path. */
-int32_t b200rwkv_debug_read(b200rwkv_engine*, const char* name, float* out, size_t cap);
+/* Test aid: copy a named internal activation buffer of the most recent internal step of b200rwkv_infer to the host as f32
+ * row-major [*rows_out, cols]; returns the column count (negative status on error).  rows = the step's tokens, or its output
+ * rows for the head's operand "a_head".  A16 operands of a split-operand step (precision 1) are returned as hi + lo.  Not on
+ * the product path. */
+int32_t b200rwkv_debug_read(b200rwkv_engine*, const char* name, float* out, size_t cap, int32_t* rows_out);
+
+/* Test aid: the projection launches a step of `mt` token tiles (1, 2, 4, 8) runs for layer `layer` (-1 = the head, at `mt`
+ * output-row tiles), in stream order.  One record of B200RWKV_PLAN_INTS int32 per launch:
+ *   [0] grid the step launches  [1] grid  [2] grid_wide  [3] total_blocks  [4] max_contrib  [5] qtype (0 f16, 1 Int8, 2 NF4)
+ *   [6] 1 = grid fixed by a static split-K  [7] nseg, then per segment (up to 8) five ints: KB, tiles, N, out_mode, act.
+ * CTA c of a launch streams the 128 x 128 blocks [c * total_blocks / grid, (c + 1) * total_blocks / grid) of the launch's
+ * segments in order (tile-major, k blocks within a tile).  Returns the number of launches (negative status on error). */
+#define B200RWKV_PLAN_INTS 48
+int32_t b200rwkv_debug_plan(b200rwkv_engine*, int32_t layer, int32_t mt, int32_t* out, size_t cap);
 
 /* Profiling aid: raw stamp rows of the most recent b200rwkv_profile_insitu replay, one row of 512 uint64 per launch
  * (out = [launches][512]): globaltimer stamps of CTA 0 in [0..7] (entry, past griddepcontrol.wait, phase marks, exit), then

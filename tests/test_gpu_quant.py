@@ -142,8 +142,10 @@ def test_unsupported_quant_requests_fail_loudly():
 
 @pytest.mark.parametrize("qtype", [capi.QUANT_INT8, capi.QUANT_NF4])
 def test_quantised_projections_at_the_7b_layer_shape(qtype):
-    """One layer with the 7B dimensions (C = 4096, F = 14336, LoRA ranks 64 / 128): the tile counts, stream-K cuts and split-K
-    slices of the BASELINE shape, batch 16, against the oracle on the dequantised weights."""
+    """One layer with the 7B dimensions (C = 4096, F = 14336, LoRA ranks 64 / 128): the tile counts and split-K slices of the
+    BASELINE shape, batch 16, against the oracle on the dequantised weights.  Every quantised launch of this shape runs whole
+    tiles per CTA (only the f16 head is cut); the quantised fix-up of cut tiles runs at the 3B width in
+    tests/test_gpu_projections.py."""
     import dataclasses
     shp = dataclasses.replace(synth.PRESETS["v6-7b"], L=1, V=4096)
     st = synth.make_st(shp, 0)
