@@ -17,6 +17,7 @@ LIB_PATH = os.path.join(_HERE, "libb200rwkv.so")
 OK = 0
 ERR_INVALID, ERR_UNSUPPORTED, ERR_CUDA, ERR_STATE = -1, -2, -3, -4
 OPTION_LAST, OPTION_FULL, OPTION_NONE = 0, 1, 2
+OPTION_SCORE, OPTION_SCORE_KEPT = 3, 4      # b200rwkv_infer_score only
 TP_HANDLE_BYTES = 128
 PLAN_INTS = 48            # B200RWKV_PLAN_INTS: one b200rwkv_debug_plan record
 
@@ -63,6 +64,7 @@ SYMBOLS = [
     ("b200rwkv_destroy", None, [_P]),
     ("b200rwkv_get_info", C.c_int32, [_P, C.POINTER(Info)]),
     ("b200rwkv_infer", C.c_int32, [_P, C.c_int32, _P, _P, _P, _P, _P, C.c_size_t, _P]),
+    ("b200rwkv_infer_score", C.c_int32, [_P, C.c_int32, _P, _P, _P, _P, _P, C.c_size_t, _P, _P, C.c_size_t]),
     ("b200rwkv_state_shape", C.c_int32, [_P, C.POINTER(C.c_int64 * 4)]),
     ("b200rwkv_state_init", C.c_int32, [_P, _P]),
     ("b200rwkv_state_load", C.c_int32, [_P, C.c_int32, _P]),

@@ -385,7 +385,9 @@ struct Profiler {
     std::vector<Rec> recs;
 };
 
-struct Snapshot { float* buf = nullptr; float* logits = nullptr; size_t bytes = 0; };   // CachedItem {state, output} on the device (run.rs:199-205)
+// CachedItem {state, output} on the device (run.rs:199-205).  `row`: the slot had a kept logits row when the snapshot was taken;
+// recorded on every tensor-parallel rank (only rank 0 holds the row itself) so that checks of it agree across ranks.
+struct Snapshot { float* buf = nullptr; float* logits = nullptr; size_t bytes = 0; bool row = false; };
 
 }  // namespace b200
 
@@ -491,6 +493,16 @@ struct b200rwkv_engine {
                      const uint32_t* allow_bits, const int32_t* bias_off, const uint32_t* bias_tok, const float* bias_val,
                      int top_k, uint32_t* ids_out, float* probs_out);
 
+    // scoring (b200rwkv_infer_score, rank 0): (row, target, destination) lists travel in their own pinned ring, separate
+    // from the step metadata; log-probabilities collect in d_logp and go to the host once per call
+    static constexpr int SCORE_RING = 4;
+    ScoreItem *h_score = nullptr, *d_score = nullptr;
+    int score_cap = 0;                       // items per ring buffer: max(maxT, S)
+    cudaEvent_t score_ev[SCORE_RING] = {nullptr, nullptr, nullptr, nullptr};
+    float* d_logp = nullptr;
+    size_t logp_floats = 0;
+    void enqueue_score(const std::vector<ScoreItem>& items, int seq);
+
     std::mutex mu, sm_mu;
 
     // LoRA files blended into the projection weights while they are uploaded (borrowed during build only)
@@ -547,7 +559,7 @@ struct b200rwkv_engine {
     int fill_meta(int* m, const std::vector<int>& slots, const std::vector<int>& counts, const std::vector<const uint32_t*>& toks,
                   const std::vector<int>& outmode /*0 none,1 last,2 full*/, int* R_out);
     void infer(int nslot, const int32_t* slot, const int32_t* ntok, const uint32_t* tokens, const int32_t* option,
-               float* logits_out, size_t cap, int32_t* rows_out);
+               float* logits_out, size_t cap, int32_t* rows_out, float* logp_out = nullptr, size_t logp_cap = 0, bool scoring = false);
     void state_xform(int slot, bool import, float* snap = nullptr);
 };
 
@@ -565,6 +577,10 @@ b200rwkv_engine::~b200rwkv_engine() {
     if (h_meta) cudaFreeHost(h_meta);
     if (tk_dev) cudaFree(tk_dev);
     if (tk_host) cudaFreeHost(tk_host);
+    if (h_score) cudaFreeHost(h_score);
+    if (d_score) cudaFree(d_score);
+    if (d_logp) cudaFree(d_logp);
+    for (auto& ev : score_ev) if (ev) cudaEventDestroy(ev);
     if (step_done) cudaEventDestroy(step_done);
     for (auto& ev : meta_ev) if (ev) cudaEventDestroy(ev);
     if (d_hidden_all) cudaFree(d_hidden_all);
@@ -1556,26 +1572,73 @@ int b200rwkv_engine::fill_meta(int* m, const std::vector<int>& slots, const std:
     return T;
 }
 
+void b200rwkv_engine::enqueue_score(const std::vector<ScoreItem>& items, int seq) {
+    // pinned ring: a host buffer is rewritten only after the copy that read it has completed; the device list is reused in
+    // stream order
+    const int rb = seq % SCORE_RING;
+    if (seq >= SCORE_RING) CK(cudaEventSynchronize(score_ev[rb]));
+    ScoreItem* h = h_score + (size_t)rb * score_cap;
+    memcpy(h, items.data(), items.size() * sizeof(ScoreItem));
+    CK(cudaMemcpyAsync(d_score, h, items.size() * sizeof(ScoreItem), cudaMemcpyHostToDevice, stream));
+    CK(cudaEventRecord(score_ev[rb], stream));
+    ScoreParams sp;
+    memset(&sp, 0, sizeof(sp));
+    for (int q = 0; q < world; ++q) sp.shard[q] = (const float*)(peer_base[q] + off_logits);
+    sp.world = world; sp.Vl = Vl; sp.V = V;
+    sp.keep = d_keep; sp.items = d_score; sp.logp = d_logp;
+    score_rows_kernel<<<(unsigned)items.size(), SCORE_THREADS, 0, stream>>>(sp);
+    CK(cudaGetLastError());
+    ++launch_total;
+}
+
 void b200rwkv_engine::infer(int nslot, const int32_t* slot, const int32_t* ntok, const uint32_t* tokens, const int32_t* option,
-                            float* logits_out, size_t cap, int32_t* rows_out) {
+                            float* logits_out, size_t cap, int32_t* rows_out, float* logp_out, size_t logp_cap, bool scoring) {
     REQUIRE(nslot >= 0 && (nslot == 0 || (slot && ntok && option)), B200RWKV_ERR_INVALID, "infer: null argument");
     REQUIRE(connected, B200RWKV_ERR_INVALID, "tensor-parallel engine is not connected (b200rwkv_tp_connect)");
+    // SCORE / SCORE_KEPT entries (b200rwkv_infer_score only) step like FULL; their rows are scored on the device, not copied
+    const int opt_max = scoring ? B200RWKV_OPTION_SCORE_KEPT : B200RWKV_OPTION_NONE;
+    auto is_score = [&](int i) { return option[i] == B200RWKV_OPTION_SCORE || option[i] == B200RWKV_OPTION_SCORE_KEPT; };
     std::vector<char> seen(S, 0);
-    size_t total_rows = 0, total_tok = 0;
+    size_t total_rows = 0, total_tok = 0, total_score = 0;
     for (int i = 0; i < nslot; ++i) {
         REQUIRE(slot[i] >= 0 && slot[i] < S, B200RWKV_ERR_STATE, "infer: slot out of range");
         REQUIRE(!seen[slot[i]], B200RWKV_ERR_INVALID, "infer: duplicate slot in one call");
         seen[slot[i]] = 1;
         REQUIRE(ntok[i] >= 0, B200RWKV_ERR_INVALID, "infer: negative token count");
-        REQUIRE(option[i] >= B200RWKV_OPTION_LAST && option[i] <= B200RWKV_OPTION_NONE, B200RWKV_ERR_INVALID, "infer: bad option");
+        REQUIRE(option[i] >= B200RWKV_OPTION_LAST && option[i] <= opt_max, B200RWKV_ERR_INVALID, "infer: bad option");
         const int r = (option[i] == B200RWKV_OPTION_FULL) ? ntok[i] : ((option[i] == B200RWKV_OPTION_LAST && ntok[i] > 0) ? 1 : 0);
         if (rows_out) rows_out[i] = r;
         total_rows += (size_t)r;
         total_tok += (size_t)ntok[i];
+        if (is_score(i)) total_score += (size_t)ntok[i];
     }
+    for (int i = 0; i < nslot; ++i) {
+        if (option[i] != B200RWKV_OPTION_SCORE_KEPT) continue;
+        REQUIRE(Vl % 4 == 0, B200RWKV_ERR_UNSUPPORTED, "infer_score: this engine keeps no logits rows (num_vocab / world is not a multiple of 4)");
+        std::lock_guard<std::mutex> lk(keep_mu);
+        REQUIRE(keep_valid[slot[i]], B200RWKV_ERR_STATE, "infer_score: SCORE_KEPT on slot " + std::to_string(slot[i]) + ", which has no kept logits row");
+    }
+    // tensor parallel: rank 0 writes logp_out; another rank checks it only when given it (in-process ranks all are)
+    if (total_score > 0 && (rank == 0 || logp_out))
+        REQUIRE(logp_out && logp_cap >= total_score, B200RWKV_ERR_INVALID, "infer_score: logp buffer missing or too small");
     REQUIRE(total_tok == 0 || tokens, B200RWKV_ERR_INVALID, "infer: null tokens");
     for (size_t i = 0; i < total_tok; ++i)
         REQUIRE(tokens[i] < (uint32_t)V, B200RWKV_ERR_INVALID, "infer: token id " + std::to_string(tokens[i]) + " is outside the vocabulary");
+    const bool do_score = total_score > 0 && rank == 0;
+    if (do_score) {
+        if (!h_score) {
+            score_cap = std::max(maxT, S);
+            CK(cudaMallocHost(&h_score, (size_t)SCORE_RING * score_cap * sizeof(ScoreItem)));
+            d_score = (ScoreItem*)dalloc((size_t)score_cap * sizeof(ScoreItem));
+            for (auto& ev : score_ev) CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+        }
+        if (total_score > logp_floats) {
+            if (d_logp) { CK(cudaFree(d_logp)); d_logp = nullptr; logp_floats = 0; }
+            const size_t want = std::max<size_t>(total_score, 4096);
+            CK(cudaMalloc(&d_logp, want * 4));
+            logp_floats = want;
+        }
+    }
     const bool want_logits = (rank == 0);          // tensor parallel: rank 0 gathers all vocabulary shards
     REQUIRE(!want_logits || !logits_out || total_rows * (size_t)V <= cap || total_rows == 0, B200RWKV_ERR_INVALID, "infer: logits buffer too small");
     // logits_out == NULL: the rows stay in HBM (b200rwkv_sample_topk reads the last row of every slot from there)
@@ -1591,6 +1654,19 @@ void b200rwkv_engine::infer(int nslot, const int32_t* slot, const int32_t* ntok,
         base[i + 1] = base[i] + (size_t)ntok[i];
         const int r = (option[i] == B200RWKV_OPTION_FULL) ? ntok[i] : ((option[i] == B200RWKV_OPTION_LAST && ntok[i] > 0) ? 1 : 0);
         row_base[i + 1] = row_base[i] + (size_t)r;
+    }
+    std::vector<size_t> lbase(nslot + 1, 0);      // where each scoring entry's log-probabilities start in logp_out
+    for (int i = 0; i < nslot; ++i) lbase[i + 1] = lbase[i] + (is_score(i) ? (size_t)ntok[i] : 0);
+    int score_seq = 0;
+    if (do_score) {
+        // first token of a SCORE_KEPT entry: scored against the slot's kept row as it stands before any step of this call
+        std::vector<ScoreItem> first;
+        for (int i = 0; i < nslot; ++i)
+            if (option[i] == B200RWKV_OPTION_SCORE_KEPT && ntok[i] > 0) first.push_back({-(slot[i] + 1), tokens[base[i]], (int)lbase[i], 0});
+        if (!first.empty()) {
+            std::lock_guard<std::mutex> lk(keep_mu);
+            enqueue_score(first, score_seq++);
+        }
     }
     if (hidden_keep && total_tok > hidden_cap_rows) {
         if (d_hidden_all) { CK(cudaFree(d_hidden_all)); d_hidden_all = nullptr; hidden_cap_rows = 0; }
@@ -1629,7 +1705,7 @@ void b200rwkv_engine::infer(int nslot, const int32_t* slot, const int32_t* ntok,
             s_slots.push_back(slot[i]);
             s_toks.push_back(tokens + base[i] + pos[i]);
             const bool finishes = (pos[i] + s_counts[j] == ntok[i]);
-            s_out.push_back(option[i] == B200RWKV_OPTION_FULL ? 2 : ((finishes && option[i] == B200RWKV_OPTION_LAST) ? 1 : 0));
+            s_out.push_back((option[i] == B200RWKV_OPTION_FULL || is_score(i)) ? 2 : ((finishes && option[i] == B200RWKV_OPTION_LAST) ? 1 : 0));
         }
         // pinned metadata ring: a buffer is rewritten only after the copy that read it has completed
         const int mb = step_no % META_RING;
@@ -1642,6 +1718,22 @@ void b200rwkv_engine::infer(int nslot, const int32_t* slot, const int32_t* ntok,
         CK(cudaMemcpyAsync(d_meta, hm, meta_ints * 4, cudaMemcpyHostToDevice, stream));
         CK(cudaEventRecord(meta_ev[mb], stream));
         run_step(mt_bucket(T), R > 0 ? mt_bucket(R) : 0);
+        if (do_score) {
+            // the target of a row is the next token of the same entry -- the first token of the entry's next step when the
+            // packer cut its run here; an entry's last row has none.  Launched after the step, outside its graph.
+            std::vector<ScoreItem> items;
+            int r0 = 0;
+            for (size_t j = 0; j < s_entry.size(); ++j) {
+                const int i = s_entry[j];
+                if (is_score(i))
+                    for (int k = 0; k < s_counts[j]; ++k) {
+                        const size_t p = (size_t)pos[i] + k;
+                        if (p + 1 < (size_t)ntok[i]) items.push_back({r0 + k, tokens[base[i] + p + 1], (int)(lbase[i] + p + 1), 0});
+                    }
+                r0 += s_out[j] == 2 ? s_counts[j] : (s_out[j] == 1 ? 1 : 0);
+            }
+            if (!items.empty()) enqueue_score(items, score_seq++);
+        }
         if (hidden_keep) {       // hidden rows of every token of this call (b200rwkv_last_hidden), in entry order
             int t0 = 0;
             for (size_t j = 0; j < s_entry.size(); ++j) {
@@ -1664,6 +1756,7 @@ void b200rwkv_engine::infer(int nslot, const int32_t* slot, const int32_t* ntok,
             size_t j = 0;
             while (j < s_entry.size()) {
                 const int i = s_entry[j];
+                if (is_score(i)) { r0 += s_counts[j]; ++j; continue; }     // scored on the device, never copied
                 int nr = s_out[j] == 2 ? s_counts[j] : (s_out[j] == 1 ? 1 : 0);
                 if (nr == 0) { ++j; continue; }
                 const size_t dst = row_base[i] + (size_t)rows_done[i];
@@ -1672,6 +1765,7 @@ void b200rwkv_engine::infer(int nslot, const int32_t* slot, const int32_t* ntok,
                 size_t k = j + 1;
                 while (k < s_entry.size()) {
                     const int i2 = s_entry[k];
+                    if (is_score(i2)) break;                                  // its rows sit between: the source run ends
                     const int nr2 = s_out[k] == 2 ? s_counts[k] : (s_out[k] == 1 ? 1 : 0);
                     if (nr2 == 0) { ++k; continue; }
                     if (row_base[i2] + (size_t)rows_done[i2] != dst + (size_t)run) break;
@@ -1694,7 +1788,11 @@ void b200rwkv_engine::infer(int nslot, const int32_t* slot, const int32_t* ntok,
         for (size_t j = 0; j < s_entry.size(); ++j) pos[s_entry[j]] += s_counts[j];
         ++step_no;
     }
+    if (do_score) CK(cudaMemcpyAsync(logp_out, d_logp, total_score * 4, cudaMemcpyDeviceToHost, stream));
     CK(cudaStreamSynchronize(stream));
+    if (do_score)
+        for (int i = 0; i < nslot; ++i)
+            if (option[i] == B200RWKV_OPTION_SCORE && ntok[i] > 0) logp_out[lbase[i]] = NAN;     // x0 has no preceding row
     if (hidden_keep) hidden_rows = (int)total_tok;
 }
 
@@ -2053,12 +2151,13 @@ int32_t b200rwkv_get_info(b200rwkv_engine* e, b200rwkv_info* out) {
 }
 
 static int32_t rank_infer(b200rwkv_engine* e, int32_t nslot, const int32_t* slot, const int32_t* ntok, const uint32_t* tokens,
-                       const int32_t* option, float* logits_out, size_t logits_cap, int32_t* rows_out) {
+                       const int32_t* option, float* logits_out, size_t logits_cap, int32_t* rows_out, float* logp_out = nullptr,
+                       size_t logp_cap = 0, bool scoring = false) {
     API_BEGIN(e)
     REQUIRE(e, B200RWKV_ERR_INVALID, "null engine");
     std::lock_guard<std::mutex> lk(e->mu);
     CK(cudaSetDevice(e->dev));
-    e->infer(nslot, slot, ntok, tokens, option, logits_out, logits_cap, rows_out);
+    e->infer(nslot, slot, ntok, tokens, option, logits_out, logits_cap, rows_out, logp_out, logp_cap, scoring);
     API_END
 }
 
@@ -2138,12 +2237,14 @@ static int32_t rank_state_read(b200rwkv_engine* e, int32_t slot, uint64_t* snaps
     REQUIRE(slot >= 0 && slot < e->S, B200RWKV_ERR_STATE, "slot out of range");
     std::lock_guard<std::mutex> lk(e->mu);
     CK(cudaSetDevice(e->dev));
-    bool has_row;
+    bool row, has_row;
     {
         std::lock_guard<std::mutex> lk2(e->keep_mu);
-        has_row = e->d_keep && e->keep_valid[slot];
+        row = e->keep_valid[slot];
+        has_row = e->d_keep && row;
     }
     Snapshot sn = snapshot_alloc(e, has_row);
+    sn.row = row;
     try {
         snapshot_copy(e, slot, sn.buf, true);
         // the slot's last logits row travels with the state (CachedItem.output, run.rs:199-205): a cache hit can be sampled
@@ -2176,7 +2277,7 @@ static int32_t rank_state_write(b200rwkv_engine* e, int32_t slot, uint64_t snaps
     CK(cudaStreamSynchronize(e->stream));
     {
         std::lock_guard<std::mutex> lk2(e->keep_mu);
-        e->keep_valid[slot] = (e->d_keep && it->second.logits) ? 1 : 0;
+        e->keep_valid[slot] = it->second.row ? 1 : 0;       // rank 0: the snapshot holds the row exactly when `row` is set
     }
     API_END
 }
@@ -2221,6 +2322,7 @@ static int32_t rank_snapshot_load(b200rwkv_engine* e, const float* state_in, con
     std::lock_guard<std::mutex> lk(e->mu);
     CK(cudaSetDevice(e->dev));
     Snapshot sn = snapshot_alloc(e, logits_in != nullptr && e->d_keep != nullptr);
+    sn.row = logits_in != nullptr;
     try {
         const size_t n = (size_t)e->L * (e->N + 2) * e->C;
         CK(cudaMemcpyAsync(e->d_api, state_in, n * 4, cudaMemcpyHostToDevice, e->stream));
@@ -2942,6 +3044,13 @@ int32_t b200rwkv_infer(b200rwkv_engine* e, int32_t nslot, const int32_t* slot, c
     return RANKS(e, rank_infer(er, nslot, slot, ntok, tokens, option, r_ == 0 ? logits_out : nullptr, r_ == 0 ? logits_cap : 0,
                                r_ == 0 ? rows_out : nullptr));
 }
+int32_t b200rwkv_infer_score(b200rwkv_engine* e, int32_t nslot, const int32_t* slot, const int32_t* ntok, const uint32_t* tokens,
+                             const int32_t* option, float* logits_out, size_t logits_cap, int32_t* rows_out, float* logp_out,
+                             size_t logp_cap) {
+    // every in-process rank is handed logp_out so that its argument checks agree with rank 0's; only rank 0 writes it
+    return RANKS(e, rank_infer(er, nslot, slot, ntok, tokens, option, r_ == 0 ? logits_out : nullptr, r_ == 0 ? logits_cap : 0,
+                               r_ == 0 ? rows_out : nullptr, logp_out, logp_cap, true));
+}
 int32_t b200rwkv_state_load(b200rwkv_engine* e, int32_t slot, const float* in) { return RANKS(e, rank_state_load(er, slot, in)); }
 
 // head-sharded state: every rank exports the WKV rows of its own heads (zeros elsewhere); the shift rows are replicated
@@ -2992,7 +3101,8 @@ int32_t b200rwkv_snapshot_back(b200rwkv_engine* e, uint64_t id, float* state_out
 int32_t b200rwkv_snapshot_load(b200rwkv_engine* e, const float* state_in, const float* logits_in, uint64_t* snapshot_id) {
     if (!e || !e->group) return rank_snapshot_load(e, state_in, logits_in, snapshot_id);
     std::vector<uint64_t> ids(e->group->ranks.size(), 0);
-    const int32_t st = e->group->spmd([&](int r) { return rank_snapshot_load(e->group->ranks[r], state_in, r == 0 ? logits_in : nullptr, &ids[r]); });
+    // every rank records whether a row came with the state; only rank 0 keeps rows and reads logits_in
+    const int32_t st = e->group->spmd([&](int r) { return rank_snapshot_load(e->group->ranks[r], state_in, logits_in, &ids[r]); });
     if (st < 0) return st;
     for (uint64_t id : ids)
         if (id != ids[0]) { g_err = "internal: snapshot ids diverged across ranks"; return B200RWKV_ERR_STATE; }

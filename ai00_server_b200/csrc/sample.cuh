@@ -211,4 +211,75 @@ __global__ void __launch_bounds__(KEEP_THREADS) keep_rows_kernel(const __grid_co
     }
 }
 
+// ---------------------------------------------------------------------------------------
+// Scoring given tokens (b200rwkv_infer_score): logp = x[t] - m - log sum exp(x - m) of one logits row at one target id, for
+// a list of (source row, target, destination).  This is the reference's perplexity() (crates/ai00-core/src/run.rs:699-755),
+// which copies every row to the host and normalises it there only to read back one number.
+// One CTA per row: each thread keeps an online (max, sum exp) over its strided share of the row (L2 resident, read once),
+// then warps and the block combine the pairs in a fixed order -- no float atomics, so the result is bit-reproducible.
+// Sources: a row of this step's logits (tensor parallel: rank 0 reads the vocabulary shard of every rank, complete after the
+// step's last rendezvous), or keep[slot] (already gathered) for the first token of a SCORE_KEPT entry.
+// ---------------------------------------------------------------------------------------
+struct ScoreItem {
+    int src;                    // >= 0: output row of the step;  < 0: keep[-src - 1]
+    unsigned target;            // token id whose log-probability is wanted
+    int dst;                    // index into logp
+    int pad;
+};
+struct ScoreParams {
+    const float* shard[8];      // [R][Vl] logits shard of every rank (peer mapped)
+    int world, Vl, V;
+    const float* keep;          // [S][V]
+    const ScoreItem* items;     // [gridDim.x]
+    float* logp;
+};
+constexpr int SCORE_THREADS = 512;
+
+__device__ __forceinline__ void lse_push(float& m, float& s, const float x) {
+    if (x > m) { s = s * expf(m - x) + 1.f; m = x; }
+    else s += expf(x - m);
+}
+__device__ __forceinline__ void lse_merge(float& m, float& s, const float m2, const float s2) {
+    const float M = fmaxf(m, m2);
+    if (M == -INFINITY) return;                      // both halves empty
+    s = s * expf(m - M) + s2 * expf(m2 - M);         // commutative: both lanes of a butterfly agree bit for bit
+    m = M;
+}
+
+__global__ void __launch_bounds__(SCORE_THREADS) score_rows_kernel(const __grid_constant__ ScoreParams p) {
+    __shared__ float red_m[SCORE_THREADS / 32], red_s[SCORE_THREADS / 32];
+    const ScoreItem it = p.items[blockIdx.x];
+    const bool kept = it.src < 0;
+    const int nsh = kept ? 1 : p.world, w = kept ? p.V : p.Vl;
+    float m = -INFINITY, s = 0.f;
+    for (int q = 0; q < nsh; ++q) {
+        const float* row = kept ? p.keep + (size_t)(-it.src - 1) * p.V : p.shard[q] + (size_t)it.src * p.Vl;
+        if ((w & 3) == 0) {
+            const float4* r4 = reinterpret_cast<const float4*>(row);
+            for (int i = threadIdx.x; i < (w >> 2); i += SCORE_THREADS) {
+                const float4 v = __ldcg(r4 + i);
+                lse_push(m, s, v.x); lse_push(m, s, v.y); lse_push(m, s, v.z); lse_push(m, s, v.w);
+            }
+        } else {
+            for (int i = threadIdx.x; i < w; i += SCORE_THREADS) lse_push(m, s, __ldcg(row + i));
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) lse_merge(m, s, __shfl_xor_sync(0xffffffffu, m, o), __shfl_xor_sync(0xffffffffu, s, o));
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (lane == 0) { red_m[warp] = m; red_s[warp] = s; }
+    __syncthreads();
+    if (warp != 0) return;
+    m = lane < SCORE_THREADS / 32 ? red_m[lane] : -INFINITY;
+    s = lane < SCORE_THREADS / 32 ? red_s[lane] : 0.f;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) lse_merge(m, s, __shfl_xor_sync(0xffffffffu, m, o), __shfl_xor_sync(0xffffffffu, s, o));
+    if (lane == 0) {
+        const int tq = kept ? 0 : (int)(it.target / (unsigned)p.Vl);
+        const float* row = kept ? p.keep + (size_t)(-it.src - 1) * p.V : p.shard[tq] + (size_t)it.src * p.Vl;
+        const float xt = __ldcg(row + (kept ? it.target : it.target - (unsigned)tq * p.Vl));
+        p.logp[it.dst] = (xt - m) - logf(s);
+    }
+}
+
 }  // namespace b200

@@ -313,6 +313,77 @@ class Model:
             off += r
         return res
 
+    # ---- scoring: b200rwkv_infer_score ----
+    def infer_score(self, slots, ntok, tokens, options, out: np.ndarray | None = None):
+        """One b200rwkv_infer_score call.  Options as infer_raw plus capi.OPTION_SCORE / OPTION_SCORE_KEPT.  Returns (host rows
+        per entry -- [rows, V], none for scoring entries --, one f32 log-probability array per scoring entry in entry order)."""
+        V = self.info["num_vocab"]
+        n = len(slots)
+        scoring = (capi.OPTION_SCORE, capi.OPTION_SCORE_KEPT)
+        total = sum(nt if o == capi.OPTION_FULL else (1 if (o == capi.OPTION_LAST and nt > 0) else 0) for nt, o in zip(ntok, options))
+        nscore = sum(nt for nt, o in zip(ntok, options) if o in scoring)
+        if out is None and total > 0:
+            out = np.empty((total, V), np.float32)
+        logp = np.empty(max(nscore, 1), np.float32)
+        a_slot, a_ntok = np.asarray(slots, np.int32), np.asarray(ntok, np.int32)
+        a_tok, a_opt = np.asarray(tokens, np.uint32), np.asarray(options, np.int32)
+        a_rows = np.zeros(max(n, 1), np.int32)
+        capi.check(capi.lib().b200rwkv_infer_score(self._h, n, capi.ptr(a_slot), capi.ptr(a_ntok), capi.ptr(a_tok), capi.ptr(a_opt),
+                                                   capi.ptr(out) if out is not None else None, out.size if out is not None else 0,
+                                                   capi.ptr(a_rows), capi.ptr(logp), nscore), self._h)
+        rows, lps, off, loff = [], [], 0, 0
+        for i in range(n):
+            r = int(a_rows[i])
+            rows.append(out[off:off + r] if r else np.zeros((0, V), np.float32))
+            off += r
+            if options[i] in scoring:
+                lps.append(logp[loff:loff + ntok[i]].copy())
+                loff += ntok[i]
+        return rows, lps
+
+    def perplexity(self, batch: int, tokens, head: bool) -> float:
+        """The reference's `perplexity(batch, tokens, head)` (run.rs:699-755) on the device: -mean ln p of the tokens, fed to
+        slot `batch` from its current state.  head = True is `Some(output[tokens[0]])`: the first token is scored against the
+        slot's kept row (SCORE_KEPT).  head = False is `None`: like the reference, token 0 is prepended and fed too, and the sum
+        of len(tokens) terms is divided by len(tokens) + 1.  The reference's f32 sum of ln p is kept."""
+        toks = [int(t) for t in tokens]
+        if not toks:
+            raise capi.B200Error(capi.ERR_INVALID, "perplexity of an empty token list is undefined (the reference never asks)")
+        if head:
+            _, (lp,) = self.infer_score([batch], [len(toks)], toks, [capi.OPTION_SCORE_KEPT])
+        else:
+            toks = [0] + toks
+            _, (lp,) = self.infer_score([batch], [len(toks)], toks, [capi.OPTION_SCORE])
+            lp = lp[1:]
+        s = np.float32(0.0)
+        for x in lp:
+            s = np.float32(s + x)
+        return float(np.float32(-s) / np.float32(len(toks)))
+
+    def choose(self, batch: int, choices, calibrate: bool, init_state: np.ndarray | None = None) -> list[float]:
+        """The Choose branch of the reference (run.rs:936-983) on slot `batch`, which holds the prompt's state and kept row:
+        ppl per choice (lower is better, empty choices +inf).  calibrate subtracts each choice's no-head perplexity from
+        `init_state` (the cached state of the request, default State::init).  The slot's state and kept row are snapshotted
+        with State::read and restored with State::write after every choice."""
+        backed = self.state.read(batch)
+        try:
+            ppl = [float("inf")] * len(choices)
+            if calibrate:
+                init = self.state.init() if init_state is None else init_state
+                for i, c in enumerate(choices):
+                    if len(c):
+                        self.state.load(init, batch)
+                        ppl[i] = -self.perplexity(batch, c, head=False)
+                self.state.write(backed, batch)
+            for i, c in enumerate(choices):
+                if len(c):
+                    p = self.perplexity(batch, c, head=True)
+                    ppl[i] = ppl[i] + p if calibrate else p
+                    self.state.write(backed, batch)
+        finally:
+            backed.free()
+        return ppl
+
     def softmax(self, tensors):
         """`softmax(&context, Vec<TensorCpu<f32>>)`: list of [V] rows in, list out."""
         if not tensors:

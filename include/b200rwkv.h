@@ -59,6 +59,9 @@ enum {
      * cut by token_chunk_size and continues in the next infer call (run.rs:1134-1145) */
     B200RWKV_OPTION_NONE = 2
 };
+/* Scoring options, accepted by b200rwkv_infer_score only (b200rwkv_infer answers B200RWKV_ERR_INVALID). */
+#define B200RWKV_OPTION_SCORE 3
+#define B200RWKV_OPTION_SCORE_KEPT 4
 
 /* Replaces `Loader::info(&SafeTensors)` — crates/ai00-core/src/lib.rs:587,
  * crates/ai00-server/src/api/file.rs:115.  Pure host code, no GPU needed. */
@@ -144,6 +147,24 @@ int32_t b200rwkv_get_info(b200rwkv_engine*, b200rwkv_info* out);
 int32_t b200rwkv_infer(b200rwkv_engine*, int32_t nslot, const int32_t* slot, const int32_t* ntok,
                        const uint32_t* tokens, const int32_t* option, float* logits_out,
                        size_t logits_cap, int32_t* rows_out);
+
+/* Replaces the forward pass of the reference's perplexity() -- crates/ai00-core/src/run.rs:699-755, run once per choice (twice
+ * with `calibrate`) by the chooses endpoint, run.rs:936-983 -- which copies one num_vocab f32 row per token to the host and
+ * normalises it there to read one number.  Same arguments and results as b200rwkv_infer, and additionally:
+ * an entry with option SCORE or SCORE_KEPT holding tokens x0 .. x{n-1} steps like FULL but copies no logits rows
+ * (rows_out[i] = 0); its last row becomes the slot's kept row, as for LAST with logits_out = NULL.  It writes n floats to
+ * `logp_out`, packed in entry order over the scoring entries only:
+ *     logp[j] = log_softmax(row of x{j-1})[x{j}]          j >= 1
+ *     logp[0] = NaN                                        SCORE
+ *     logp[0] = log_softmax(kept row at call start)[x0]    SCORE_KEPT (the reference's `head` term; chained calls are exact)
+ * `logp_cap` is in floats.  Refused before any step runs, so a refused call changes no state:
+ *     SCORE_KEPT on a slot with no kept row                             B200RWKV_ERR_STATE
+ *     logp_out == NULL with scoring entries, or logp_cap too small      B200RWKV_ERR_INVALID
+ *     SCORE_KEPT where the engine keeps no rows (num_vocab / world % 4) B200RWKV_ERR_UNSUPPORTED
+ * Tensor parallel (create_tp): SPMD like b200rwkv_infer; rank 0 fills logp_out, the other ranks may pass NULL. */
+int32_t b200rwkv_infer_score(b200rwkv_engine*, int32_t nslot, const int32_t* slot, const int32_t* ntok,
+                             const uint32_t* tokens, const int32_t* option, float* logits_out, size_t logits_cap,
+                             int32_t* rows_out, float* logp_out, size_t logp_cap);
 
 /* `State` trait object — crates/ai00-core/src/lib.rs:399,494; uses at run.rs:477,1099-1107.
  * The host-visible state of one slot is an f32 tensor of web-rwkv shape [C, N+2, L, 1]
